@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            the CUDA engine (one rank per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...  the reference's own CPU path on the host cores
   python bench.py --config single|hdr|pooled|mixed         BASELINE.json configs[1] (default) / [2] / [3] / [4]
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's outputs (seeded sample) as .npy
 
 One step = one pass of the hot path over one batch of synthetic reads, every read aligned (no dedup shortcut, so
 reads/s == DP problems/s):
@@ -424,7 +425,10 @@ def main():
     ap.add_argument("--edit-cap", type=int, default=8)
     ap.add_argument("--e2e-steps", type=int, default=10)
     ap.add_argument("--no-api", action="store_true", help="skip the process_fastq (api) leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -522,6 +526,8 @@ def main():
     launches = eng.launch_count() - launches0
     pair_items, single_items = eng.path_counts()
     L.c2b_set_pair_order(eng.h, None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, args.steps, n, R, W, args.edit_cap, d_recs, d_alns, d_str, d_ed)
 
     recs = np.frombuffer(d_recs.cpu().numpy().tobytes(), dtype=_lib.REC_DTYPE)
     alns = np.frombuffer(d_alns.cpu().numpy().tobytes(), dtype=_lib.ALN_DTYPE).reshape(n, R)
@@ -715,6 +721,44 @@ def main():
         dist.barrier()
         dist.destroy_process_group()
     return 0
+
+
+DUMP_READS = 1 << 15                             # seeded sample of the timed batch written by --dump-outputs
+DUMP_STRING_READS = 1 << 10                      # ... and the part of it whose aligned strings are written
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(dirpath, eng, steps, n, R, W, cap, d_recs, d_alns, d_str, d_ed):
+    """--dump-outputs: what a caller of c2b_align_batch_device receives after the last timed step, on a fixed seeded sample of
+    the batch's reads (the batch itself is seeded too, so two builds can be compared file for file): every field of the read
+    records and of the per-amplicon alignment records, the edit lists and the aligned strings with the unused entries zeroed,
+    and the count block divided by the number of timed steps (it accumulates over them).  float64 where a field can exceed
+    float32's exact integers."""
+    from crispresso2_b200 import _lib
+    os.makedirs(dirpath, exist_ok=True)
+    idx = np.sort(np.random.default_rng(20240).choice(n, size=min(n, DUMP_READS), replace=False))
+    recs = np.frombuffer(d_recs.cpu().numpy().tobytes(), dtype=_lib.REC_DTYPE)[idx]
+    alns = np.frombuffer(d_alns.cpu().numpy().tobytes(), dtype=_lib.ALN_DTYPE).reshape(n, R)[idx]
+    edits = np.frombuffer(d_ed.cpu().numpy().tobytes(), dtype=_lib.EDIT_DTYPE).reshape(n, R, cap)[idx]
+    sidx = idx[:DUMP_STRING_READS]
+    strs = d_str.cpu().numpy().reshape(n, R, 2, W)[sidx].astype(np.float32)
+    out = {"read_index": idx.astype(np.float64)}
+    for f in _lib.REC_DTYPE.names:
+        out["rec_" + f] = recs[f].astype(np.float64)
+    for f in _lib.ALN_DTYPE.names:
+        out["aln_" + f] = alns[f].astype(np.float64)
+    used = np.arange(cap)[None, None, :] < np.minimum(alns["n_edits"], cap)[:, :, None]
+    for f in ("a", "b", "type", "in_window", "base"):
+        out["edit_" + f] = np.where(used, edits[f], 0).astype(np.float32)
+    cols = np.arange(W)[None, None, None, :] >= (W - alns["aln_len"][:len(sidx)].astype(np.int64))[:, :, None, None]
+    out["strings"] = np.where(cols, strs, 0).astype(np.float32)
+    out["string_read_index"] = sidx.astype(np.float64)
+    out["counts"] = eng.counts_raw().astype(np.float64) / steps
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    for name, a in out.items():
+        np.save(os.path.join(dirpath, name + ".npy"), a)
 
 
 def cpu_baseline_generic(w):

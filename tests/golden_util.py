@@ -1,5 +1,6 @@
 """Helpers shared by the parity tests: fixture loading and the reference's count-vector file layout."""
 import gzip
+import hashlib
 import json
 import os
 
@@ -78,3 +79,66 @@ def _norm(g):
 def payload_equal(want, got):
     """Compares two payloads (dict or ResultsSlotsDict-like); returns the list of differing keys."""
     return [k for k, w in want.items() if _norm(got[k]) != _norm(w)]
+
+
+def load_reference_answers():
+    """tests/golden/reference_answers.json.gz: what the reference's own functions returned for the inputs of the tests that
+    compare with it (written by tests/golden/gen_reference_answers.py)."""
+    return load("reference_answers")
+
+
+def canon(x):
+    """JSON-able form of a returned value that keeps what `==` on the original objects would see: tuple vs list, the dtype
+    kind of an array, int vs float vs bool.  Objects with a mapping or attribute interface become their items."""
+    if isinstance(x, np.ndarray):
+        return {"nd": x.dtype.kind, "v": canon(x.tolist())}
+    if isinstance(x, np.generic):
+        x = x.item()
+    if x is None or isinstance(x, (bool, int, float, str)):
+        return x
+    if isinstance(x, tuple):
+        return {"t": [canon(v) for v in x]}
+    if isinstance(x, list):
+        return [canon(v) for v in x]
+    if isinstance(x, dict):
+        return {"d": {str(k): canon(v) for k, v in x.items()}}
+    if hasattr(x, "keys"):
+        return {"d": {str(k): canon(x[k]) for k in x.keys()}}
+    if hasattr(x, "__dict__"):
+        return {"d": {str(k): canon(v) for k, v in vars(x).items()}}
+    raise TypeError("no canonical form for %r" % type(x))
+
+
+def digest(x):
+    """Short hash of canon(x) (bytes are hashed as they are)."""
+    raw = x if isinstance(x, bytes) else json.dumps(canon(x), sort_keys=True).encode()
+    return hashlib.sha256(raw).hexdigest()[:16]
+
+
+def encode_value(x, arrays):
+    """canon() that can be decoded back into call arguments; arrays are stored once in `arrays` and referenced by digest."""
+    if isinstance(x, np.ndarray):
+        key = digest(x.tobytes() + str((x.dtype.str, x.shape)).encode())
+        arrays[key] = {"dtype": x.dtype.str, "shape": list(x.shape), "v": x.ravel().tolist()}
+        return {"array": key}
+    if isinstance(x, tuple):
+        return {"t": [encode_value(v, arrays) for v in x]}
+    if isinstance(x, list):
+        return [encode_value(v, arrays) for v in x]
+    if isinstance(x, dict):
+        return {"d": {str(k): encode_value(v, arrays) for k, v in x.items()}}
+    return canon(x)
+
+
+def decode_value(x, arrays):
+    if isinstance(x, list):
+        return [decode_value(v, arrays) for v in x]
+    if isinstance(x, dict):
+        if "array" in x:
+            a = arrays[x["array"]]
+            return np.array(a["v"], dtype=np.dtype(a["dtype"])).reshape(a["shape"])
+        if "t" in x:
+            return tuple(decode_value(v, arrays) for v in x["t"])
+        if "d" in x:
+            return {k: decode_value(v, arrays) for k, v in x["d"].items()}
+    return x

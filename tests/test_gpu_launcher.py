@@ -1,5 +1,5 @@
 """The shipped launcher (crispresso2_b200/launcher.py) against the UNMODIFIED reference CLI on a real GPU: the reference's own
-`CRISPResso` main() (baseline/_ref, pip-installed from /root/reference by __graft_entry__.build(); it travels to the GPU box) is
+`CRISPResso` main() (baseline/_ref, installed by the recipe in baseline/ref_shim.py; skipped where it is absent) is
 run twice on the same FASTQ -- as it is (CPU), and through `python -m crispresso2_b200.launcher` (process_fastq, filterFastqs
 and the table around the cut re-bound to the engine, sm_100a library) -- and every file of the two output folders must be
 byte-identical (SURVEY.md Appendix B).  The CPU twin of this test (warp-emulator engine) is tests/test_cli_dropin.py."""

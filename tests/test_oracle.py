@@ -1,5 +1,6 @@
 """Pins the CPU oracle (oracle/) against the reference: restated known-answer tests, golden vectors produced
-by the compiled reference (tests/golden/gen_golden.py), and -- when oracle/_ref is present -- live fuzzing."""
+by the compiled reference (tests/golden/gen_golden.py), and seeded fuzzing against the compiled reference's answers for the
+same inputs (tests/golden/gen_reference_answers.py)."""
 import gzip
 import json
 import os
@@ -104,14 +105,10 @@ def test_whole_path_golden(case, ednafull):
             assert (nf[b] == vec[r]["all_base_count_" + b]).all(), (r, b)
 
 
-# ---- live fuzz against the compiled reference (this container only) ---------------------------------------
-def test_live_fuzz_against_compiled_reference(ednafull):
-    mods = O.ref_modules()
-    if mods is None:
-        pytest.skip("oracle/_ref not built")
-    A, R = mods
+# ---- seeded fuzz against the compiled reference's answers --------------------------------------------------
+def live_fuzz_cases():
+    """-> (read, ref, gap_incentive, gap_open, gap_extend, include_idxs) of the fuzz, seeded."""
     rng = random.Random(7)
-    m = np.ascontiguousarray(ednafull)
     for _ in range(400):
         I = rng.choice([4, 9, 30, 77, 150])
         ref = "".join(rng.choice("ACGT") for _ in range(I))
@@ -123,25 +120,32 @@ def test_live_fuzz_against_compiled_reference(ednafull):
         gi = Z(I + 1)
         gi[rng.randrange(I + 1)] = 1
         go, ge = rng.choice([(-20, -2), (-1, -1), (-7, -3)])
-        want = A.global_align(read, ref, matrix=m, gap_incentive=gi, gap_open=go, gap_extend=ge)
-        assert O.global_align(read, ref, m, gi, go, ge) == want
         inc = sorted(rng.sample(range(I), min(I, 3)))
-        w = R.find_indels_substitutions(want[0], want[1], inc).__dict__
-        g = O.find_indels_substitutions(want[0], want[1], inc)
-        assert not G.payload_equal({k: (v.tolist() if hasattr(v, "tolist") else v) for k, v in w.items()}, g)
+        yield read, ref, gi, go, ge, inc
 
 
-def test_legacy_classification_restatement_against_compiled_reference():
-    """oracle.find_indels_substitutions_legacy (checker for a future device path) == the reference's compiled function on real
-    alignments (random reads aligned by the reference's own global_align)."""
-    mods = O.ref_modules()
-    if mods is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    A, R = mods
-    import random
-    rng = random.Random(5)
-    m = A.make_matrix()
+def payload_digest(p, keys):
+    """digest of the payload fields `keys`, compared as golden_util.payload_equal compares them"""
+    return G.digest({k: G._norm(p[k]) for k in keys})
+
+
+def test_live_fuzz_against_compiled_reference(ednafull):
+    gold = G.load_reference_answers()
+    wants, keys = gold["oracle_fuzz"], gold["oracle_fuzz_keys"]
+    m = np.ascontiguousarray(ednafull)
     n = 0
+    for (read, ref, gi, go, ge, inc), want in zip(live_fuzz_cases(), wants):
+        got = O.global_align(read, ref, m, gi, go, ge)
+        assert G.digest(got) == want[0], (read, ref, go, ge, got)
+        g = O.find_indels_substitutions(got[0], got[1], inc)
+        assert payload_digest(g, keys) == want[1], (got, inc, g)
+        n += 1
+    assert n == len(wants) > 300
+
+
+def legacy_cases():
+    """-> (read, ref, gap_incentive, include_idxs) of the legacy-classification fuzz, seeded."""
+    rng = random.Random(5)
     for _ in range(400):
         I = rng.choice([20, 41, 80, 150])
         ref = "".join(rng.choice("ACGT") for _ in range(I))
@@ -160,15 +164,26 @@ def test_legacy_classification_restatement_against_compiled_reference():
             continue
         gi = np.zeros(I + 1, dtype=np.int64)
         gi[rng.randrange(I + 1)] = 1
-        s1, s2, _ = A.global_align(read, ref, matrix=m, gap_incentive=gi, gap_open=-20, gap_extend=-2)
         inc = sorted(rng.sample(range(I), rng.randrange(0, min(I, 10))))
-        want = R.find_indels_substitutions_legacy(s1, s2, inc)
-        got = O.find_indels_substitutions_legacy(s1, s2, inc)
-        for k, v in want.items():
-            g = got[k]
-            if isinstance(v, np.ndarray):
-                assert list(v) == list(g), (k, s1, s2)
-            else:
-                assert v == g and type(v) is type(g), (k, v, g, s1, s2)
+        yield read, ref, gi, inc
+
+
+def legacy_digest(p):
+    """digest of a legacy payload: arrays by their elements, every other field by type and value"""
+    return G.digest({k: ["nd", G.canon(v.tolist())] if isinstance(v, np.ndarray) else [type(v).__name__, G.canon(v)]
+                     for k, v in p.items()})
+
+
+def test_legacy_classification_restatement_against_compiled_reference():
+    """oracle.find_indels_substitutions_legacy (checker for a future device path) == the reference's compiled function on real
+    alignments (random reads aligned by global_align, itself checked against the reference's alignment)."""
+    wants = G.load_reference_answers()["oracle_legacy"]
+    m = O.make_matrix()
+    n = 0
+    for (read, ref, gi, inc), want in zip(legacy_cases(), wants):
+        aln = O.global_align(read, ref, m, gi, -20, -2)
+        assert G.digest(aln) == want[0], (read, ref, aln)
+        got = O.find_indels_substitutions_legacy(aln[0], aln[1], inc)
+        assert legacy_digest(got) == want[1], (aln, inc, got)
         n += 1
-    assert n > 300
+    assert n == len(wants) > 300

@@ -1,24 +1,21 @@
 """get_consensus_alignment_from_pairs (CRISPRessoCORE.py:829-985), the per-column merge of the paired-end merge mode, natively
-(c2b_consensus_from_pairs via crispresso2_b200.paired): the reference's OWN unit test for it (tests/unit_tests/
-test_CRISPRessoCORE.py:27-468, run from /root/reference against the replacement) and a differential fuzz against the reference's
-Python function on random alignment pairs -- overlapping and disjoint mates, insertions in one or both, deletions, uncovered
-stretches, quality ties, leading / trailing gaps, quality strings that are too short (IndexError on both sides).
-CPU only; skipped where /root/reference is absent."""
-import importlib.util
+(c2b_consensus_from_pairs via crispresso2_b200.paired): the calls of the reference's OWN unit test for it (tests/unit_tests/
+test_CRISPRessoCORE.py:27-468) and a differential fuzz on random alignment pairs -- overlapping and disjoint mates, insertions in
+one or both, deletions, uncovered stretches, quality ties, leading / trailing gaps, quality strings that are too short
+(IndexError on both sides) -- each against what the reference's Python function returned for the same arguments, stored in
+tests/golden/reference_answers.json.gz (tests/golden/gen_reference_answers.py).  CPU only."""
 import os
 import random
 import sys
-import types
 
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not (os.path.isdir(os.path.join(REF, "tests", "unit_tests")) and
-                                     os.path.isdir(os.path.join(os.path.dirname(HERE), "oracle", "_ref", "CRISPResso2"))),
-                                reason="needs /root/reference and oracle/_ref")
 sys.path.insert(0, os.path.join(HERE, "emu"))
-sys.path.insert(0, os.path.join(HERE, "golden"))
+sys.path.insert(0, HERE)
+
+import golden_util as G  # noqa: E402
+from test_reference_unit_tests import replay  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -30,55 +27,13 @@ def consensus():
 
 
 def test_the_references_own_unit_test(consensus):
-    from crispresso2_b200 import align
-
-    class _Check:                                            # pytest_check.check as a hard assertion
-        def __enter__(self):
-            return self
-
-        def __exit__(self, *exc):
-            return False
-
-        @staticmethod
-        def equal(a, b, msg=""):
-            assert a == b, (a, b, msg)
-
-        @staticmethod
-        def is_true(x, msg=""):
-            assert x, msg
-
-        @staticmethod
-        def is_false(x, msg=""):
-            assert not x, msg
-
-    stubs = {"pytest_check": types.ModuleType("pytest_check"), "inline_snapshot": types.ModuleType("inline_snapshot")}
-    stubs["pytest_check"].check = _Check()
-    stubs["inline_snapshot"].snapshot = lambda x=None: x
-    pkg = types.ModuleType("CRISPResso2")
-    A = types.ModuleType("CRISPResso2.CRISPResso2Align")
-    A.read_matrix = align.read_matrix
-    core = types.ModuleType("CRISPResso2.CRISPRessoCORE")
-    core.get_consensus_alignment_from_pairs = consensus
-    pkg.CRISPResso2Align, pkg.CRISPRessoCORE = A, core
-    pkg.CRISPRessoShared = types.ModuleType("CRISPResso2.CRISPRessoShared")
-    pkg.CRISPRessoCOREResources = types.ModuleType("CRISPResso2.CRISPRessoCOREResources")
-    names = ["CRISPResso2", "pytest_check", "inline_snapshot"]
-    saved = {k: sys.modules.get(k) for k in names}
-    sys.modules.update({"CRISPResso2": pkg, **stubs})
-    cwd = os.getcwd()
-    os.chdir(REF)
-    try:
-        spec = importlib.util.spec_from_file_location("_ref_test_core", os.path.join(REF, "tests", "unit_tests", "test_CRISPRessoCORE.py"))
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        mod.test_get_consensus_alignment_from_pairs()
-    finally:
-        os.chdir(cwd)
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
+    gold = G.load_reference_answers()
+    calls = gold["consensus_unit"]
+    assert len(calls) >= 10
+    fns = {"get_consensus_alignment_from_pairs": consensus}
+    for call in calls:
+        why = replay(call, fns, gold["arrays"])
+        assert why is None, why
 
 
 def _random_alignment(rnd, ref, lo, hi):
@@ -106,13 +61,9 @@ def _random_alignment(rnd, ref, lo, hi):
     return "".join(s), "".join(f), q
 
 
-def test_differential_fuzz_against_the_reference_function(consensus):
-    import gen_golden as GG
-    ref_fn = GG.CRISPRessoCORE.get_consensus_alignment_from_pairs
+def fuzz_cases():
+    """The 6000 seeded argument tuples of the differential fuzz."""
     rnd = random.Random(11)
-    import contextlib
-    import io
-    n_ok = n_err = n_nocache = 0
     for it in range(6000):
         L = rnd.randint(8, 60)
         ref = "".join(rnd.choice("ACGT") for _ in range(L))
@@ -127,19 +78,27 @@ def test_differential_fuzz_against_the_reference_function(consensus):
         if rnd.random() < 0.1:
             q2 += "I" * rnd.randint(1, 5)                               # spare qualities: the gaps of a lone mate consume some
         sc1, sc2 = rnd.choice([(90.0, 80.0), (80.0, 90.0), (85.5, 85.5)])
-        try:
-            with contextlib.redirect_stdout(io.StringIO()):              # the reference prints when the amplicons disagree
-                want = ref_fn(s1, f1, sc1, q1, s2, f2, sc2, q2)
-        except IndexError:
-            want = IndexError
-        try:
-            got = consensus(s1, f1, sc1, q1, s2, f2, sc2, q2)
-        except IndexError:
-            got = IndexError
-        assert got == want, (s1, f1, q1, s2, f2, q2, sc1, sc2, got, want)
-        if want is IndexError:
+        yield (s1, f1, sc1, q1, s2, f2, sc2, q2)
+
+
+def fuzz_answer(fn, case):
+    """-> the value `fn` returns for `case`, or "IndexError" """
+    try:
+        return fn(*case)
+    except IndexError:
+        return "IndexError"
+
+
+def test_differential_fuzz_against_the_reference_function(consensus):
+    wants = G.load_reference_answers()["consensus_fuzz"]
+    assert len(wants) == 6000
+    n_ok = n_err = n_nocache = 0
+    for case, want in zip(fuzz_cases(), wants):
+        got = fuzz_answer(consensus, case)
+        assert G.digest(got) == want, (case, got)
+        if got == "IndexError":
             n_err += 1
         else:
             n_ok += 1
-            n_nocache += not want[4]
+            n_nocache += not got[4]
     assert n_ok > 3000 and n_err > 100 and n_nocache > 500, (n_ok, n_err, n_nocache)
